@@ -70,7 +70,12 @@ def parse():
     p.add_argument("--no-p2p", action="store_true")
     p.add_argument("--no-comm-bound", action="store_true")
     p.add_argument("--sweep-max-bytes", type=int, default=int(os.environ.get("BENCH_SWEEP_MAX", 1 << 30)))
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what their last step computed to DIR/<name>.npy (float32)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -175,20 +180,46 @@ def max_over_ranks(value, dist, world):
     return value
 
 
-def timed_steps(step, x, y, steps, dist, world):
-    """Device-resident inputs: exactly `steps` steps between two fences, CUDA events, max over ranks."""
+def timed_steps(step, x, y, steps, dist, world, last=None):
+    """Device-resident inputs: exactly `steps` steps between two fences, CUDA events, max over ranks.
+    If `last` is a list, what the final step returned is appended to it."""
     import torch
 
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     fence(dist, world)
     t0 = time.time()
     e0.record()
+    out = None
     for _ in range(steps):
-        step(x, y)
+        out = step(x, y)
     e1.record()
     fence(dist, world)
     t1 = time.time()
+    if last is not None:
+        last.append(out)
     return max_over_ranks(e0.elapsed_time(e1), dist, world), (t0, t1)
+
+
+DUMP_PARAM_SAMPLE = 1 << 20   # 4 MB of float32; all of ResNet-50's parameters would be 102 MB
+
+
+def dump_outputs(out_dir, model, loss):
+    """What the training step hands back to its caller, as float32 .npy files: the loss, the batch-norm running
+    statistics (every one of them) and a fixed, seeded sample of the updated parameters, whose values carry the
+    gradients the fused reduction produced.  Element order is the order of model.parameters() / model.buffers()."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, t):
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().to("cpu", torch.float32).numpy())
+
+    save("loss", loss.reshape(1))
+    save("bn_running_stats", torch.cat([b.reshape(-1).float() for b in model.buffers() if b.is_floating_point()]))
+    params = torch.cat([p.detach().reshape(-1).float() for p in model.parameters()]).cpu()
+    pick = torch.randperm(params.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_PARAM_SAMPLE].sort().values
+    save("params_sample", params[pick])
 
 
 def timed_steps_e2e(step, x_host, y_host, steps, dist, world, device):
@@ -1020,12 +1051,16 @@ def main():
     l0 = N.launch_count()
     if os.environ.get("BENCH_CUDA_PROFILER") == "1":  # ncu --profile-from-start off: capture the timed region only
         torch.cuda.profiler.start()
-    ms, win1 = timed_steps(step, x, y, args.steps, dist, world)
+    last = []
+    ms, win1 = timed_steps(step, x, y, args.steps, dist, world, last)
     if os.environ.get("BENCH_CUDA_PROFILER") == "1":
         torch.cuda.profiler.stop()
     launches = N.launch_count() - l0
     ktimes = state.kernel_times_ms()
     state.time_kernels = False
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, model, last[0])
+        log(f"outputs of the last timed step written to {args.dump_outputs}")
     log("timing end-to-end steps")
     # ---- end to end: inputs from pinned host memory every step, loss read back every step
     ms_e2e, win2, last_loss = timed_steps_e2e(step, x_host, y_host, args.steps, dist, world, device)

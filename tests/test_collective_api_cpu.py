@@ -173,9 +173,14 @@ def test_basic_apis(workers):
     with pytest.raises(RuntimeError):  # initialising the same group twice
         get(actors[0].init_group.remote(2, 0, "gloo", "default"))
     assert get(actors[0].report_gloo_availability.remote()) is True
-    assert get(actors[0].report_nccl_availability.remote()) is False  # no GPU here -> B200 backend unavailable
-    with pytest.raises(RuntimeError):
+    # the B200 backend is available exactly when the built library has a CUDA device to run on
+    assert get(actors[0].report_nccl_availability.remote()) is torch.cuda.is_available()
+    if torch.cuda.is_available():  # the group is declared; its communicator is built by the first collective
         get(actors[0].init_group.remote(2, 0, Backend.B200, "gpu_group"))
+        assert get(actors[0].report_is_group_initialized.remote("gpu_group")) is True
+    else:  # no CUDA device: refused, there is no CPU fallback
+        with pytest.raises(RuntimeError):
+            get(actors[0].init_group.remote(2, 0, Backend.B200, "gpu_group"))
 
 
 def test_backend_names():

@@ -247,41 +247,33 @@ def test_collectives_match_torch(pair, world, dtype):
     n = world * 3000
     ins = [torch.randn(n, generator=torch.Generator().manual_seed(100 + r)).to(dtype) for r in range(world)]
     stacked = torch.stack(ins)
+    # The ranks are threads of one process, so a device allocation made by one rank while another rank's kernel
+    # already waits for it can itself wait for that kernel.  Every buffer is therefore allocated in a round of its
+    # own before the collective is issued; outputs start as NaN so that an element the kernel did not write fails.
+    xs = e.run(lambda r: ins[r].cuda())
+
+    def collective(out_numel, fn):
+        outs = e.run(lambda r: torch.full((out_numel,), float("nan"), dtype=dtype, device="cuda"))
+        e.run(lambda r: fn(r, xs[r], outs[r]))
+        for c in e.comms:
+            c.check()
+        return [o.cpu() for o in outs]
+
     expect = {"MIN": stacked.min(0).values, "MAX": stacked.max(0).values}
     if world == 2:  # order-independent: exact (test_torch_tensor_dag.py:1340-1450)
         expect.update({"SUM": stacked.sum(0), "PRODUCT": stacked.prod(0), "AVG": (stacked.float().sum(0) / 2).to(dtype)})
     for op, want in expect.items():
-        def step(r):
-            x = ins[r].cuda()
-            out = torch.empty_like(x)
-            e.comms[r].allreduce(x, out, getattr(DagReduceOp, op))
-            return out.cpu()
-        for o in e.run(step):
+        for o in collective(n, lambda r, x, out: e.comms[r].allreduce(x, out, getattr(DagReduceOp, op))):
             assert torch.equal(o, want), op
     if world > 2:  # the kernels fold ranks 0..W-1 in order with fp32 accumulation: compare with exactly that
         from oracle import oracle as O
-        def step(r):
-            x = ins[r].cuda()
-            out = torch.empty_like(x)
-            e.comms[r].allreduce(x, out, DagReduceOp.SUM)
-            return out.cpu()
-        for o in e.run(step):
+        for o in collective(n, lambda r, x, out: e.comms[r].allreduce(x, out, DagReduceOp.SUM)):
             assert torch.equal(o, O.allreduce(ins))
 
-    def gather(r):
-        x = ins[r].cuda()
-        out = torch.empty(n * world, dtype=dtype, device="cuda")
-        e.comms[r].allgather(x, out)
-        return out.cpu()
-    for o in e.run(gather):
+    for o in collective(n * world, lambda r, x, out: e.comms[r].allgather(x, out)):
         assert torch.equal(o, torch.cat(ins))
 
-    def rs(r):
-        x = ins[r].cuda()
-        out = torch.empty(n // world, dtype=dtype, device="cuda")
-        e.comms[r].reducescatter(x, out, DagReduceOp.MAX)
-        return out.cpu()
-    for r, o in enumerate(e.run(rs)):
+    for r, o in enumerate(collective(n // world, lambda r, x, out: e.comms[r].reducescatter(x, out, DagReduceOp.MAX))):
         assert torch.equal(o, stacked.max(0).values[r * (n // world):(r + 1) * (n // world)])
 
 
